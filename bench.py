@@ -185,6 +185,25 @@ def cpu_reference_arm(cfg, rounds, seed=0, n_envs=1, threads=None):
 
 # --------------------------------------------------------------------------------------------- GPU arm
 _REAL_STDOUT = None
+DUMP_BUFFER_ROWS = 1 << 16
+
+
+def dump_outputs(out_dir, tr, est, ret, losses):
+    """What the last timed step handed back (per-episode estimated and true returns, per-agent losses) and what it left
+    in the trainer (the agents' packed parameters; a fixed seeded sample of the replay-buffer rows its rollout wrote),
+    as out_dir/<name>.npy in float32 / float64.  The inputs are seeded, so two builds run with the same arguments can be
+    compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = tr.n_real
+    lo, hi = (tr.t_filled - tr.block) * tr.N, tr.t_filled * tr.N
+    rows = np.random.RandomState(0).choice(hi - lo, size=min(hi - lo, DUMP_BUFFER_ROWS), replace=False)
+    idx = torch.as_tensor(lo + np.sort(rows), device=tr.dev)
+    out = dict(est_returns=est, true_returns=ret, **losses,
+               actor=tr.actor[:n], critic=tr.critic[:n], team_reward=tr.tr[:n], critic_local=tr.critic_local[:n],
+               buffer_sa=tr.sa[idx], buffer_ns=tr.ns[idx], buffer_r=tr.r[idx])
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a))
 
 
 def emit(line):
@@ -213,7 +232,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-consensus", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs; it does not apply to --impl reference")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     cfg = workload(args.workload, args.n_envs)
@@ -279,8 +304,8 @@ def main():
     tr.rollout_block()
 
     def step():
-        tr.rollout_block()
-        tr.update_round()
+        est, ret = tr.rollout_block()
+        return est, ret, tr.update_round()
 
     for _ in range(args.warmup):
         step()
@@ -293,9 +318,11 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step()
+        last = step()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tr, *last)
     ms = torch.tensor([e0.elapsed_time(e1)], device="cuda")
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -18,8 +18,8 @@ container (needs /root/reference, which does not exist on the GPU box).
                            verbatim on seeded inputs with injected fit permutations,
                            plus train_RPBCAC verbatim for 3 cooperative + 1 greedy +
                            1 faulty agent with common_reward=True (2 update rounds).
-7. ref_main_py.npz         the reference driver main.py as a compressed blob (executed unchanged by tests/test_main_gpu.py).
-6. ref_learning.npz        start weights / task / last-500-episode means of sim_data2.pkl
+7. ref_main_py.npz         the reference driver main.py as a compressed blob (executed unchanged by tests/test_main_*.py).
+6. ref_learning/*.npz      start weights / task / last-500-episode means of sim_data2.pkl
                            for the 45 published run directories (tools/learning_harness.py).
 """
 import os
@@ -391,10 +391,13 @@ def make_adversaries():
 def make_learning_fixture():
     """Start weights, task and published outcome of every run directory under simulation_results/raw_data (8 scenarios
     x H in {0,1} x seeds {100,200,300}; 45 exist): the inputs of tools/learning_harness.py and the numbers it prints next
-    to ours (README.md:31-45).  `ref_*` = mean over the last 500 episodes of sim_data2.pkl (run 2 of the published jobs)."""
+    to ours (README.md:31-45).  `ref_*` = mean over the last 500 episodes of sim_data2.pkl (run 2 of the published jobs).
+    One file per scenario (ref_learning/<scenario>.npz) keeps each fixture well under 1 MB."""
     import pandas as pd
-    out, runs = {}, []
+    os.makedirs(os.path.join(OUT, "ref_learning"), exist_ok=True)
+    n_runs = 0
     for scen in sorted(os.listdir(RAW)):
+        out, runs = {}, []
         for H in (0, 1):
             for seed in (100, 200, 300):
                 d = os.path.join(RAW, scen, f"H={H}", f"seed={seed}")
@@ -419,9 +422,11 @@ def make_learning_fixture():
                 for i in range(len(w)):
                     for k, v in flat_weights(w[i]).items():
                         out[f"{tag}/agent{i}/{k}"] = v
-    out["runs"] = np.array(runs)
-    np.savez_compressed(os.path.join(OUT, "ref_learning.npz"), **out)
-    print("learning fixture:", len(runs), "runs,", len(out), "arrays")
+        if runs:
+            out["runs"] = np.array(runs)
+            np.savez_compressed(os.path.join(OUT, "ref_learning", f"{scen}.npz"), **out)
+            n_runs += len(runs)
+    print("learning fixture:", n_runs, "runs")
 
 
 def make_main_fixture():

@@ -1,5 +1,8 @@
 """Helpers shared by the tests: load golden fixtures (tests/golden/*.npz)."""
+import hashlib
 import os
+import zlib
+
 import numpy as np
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -25,3 +28,14 @@ def agent_weights(z, prefix, n_agents=5):
 def pretrained(tag="malicious_H1_s100"):
     z = load("kat_est_returns.npz")
     return agent_weights(z, tag), z[f"{tag}/desired"], [str(x) for x in z[f"{tag}/labels"]]
+
+
+def write_reference_main(directory):
+    """The reference driver main.py out of ref_main_py.npz, checked against its stored SHA-256, as directory/main.py."""
+    z = load("ref_main_py.npz")
+    raw = zlib.decompress(z["blob"].tobytes())
+    assert hashlib.sha256(raw).hexdigest() == str(z["sha256"]) and len(raw) == int(z["n_bytes"])
+    script = os.path.join(directory, "main.py")
+    with open(script, "wb") as f:
+        f.write(raw)
+    return script

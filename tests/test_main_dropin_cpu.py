@@ -1,20 +1,20 @@
 """The unchanged reference main.py (main.py:1-121) imports and constructs everything from OUR packages
 (facade models, agent classes, Grid_World) and hands them to OUR train_RPBCAC.  No GPU is needed up to that call, so
 the training function is intercepted here; the GPU part of the contract is covered by tests/test_api_gpu.py.
-Skipped where the reference checkout is absent (e.g. on the GPU box)."""
+The driver comes out of tests/golden/ref_main_py.npz (byte-identical, SHA-256 checked)."""
 import os
 import sys
 
 import numpy as np
 import pandas as pd
-import pytest
+
+from golden_util import write_reference_main
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_MAIN = os.environ.get("RCMARL_REFERENCE", "/root/reference") + "/main.py"
 
 
-@pytest.mark.skipif(not os.path.exists(REF_MAIN), reason="reference checkout not present")
 def test_reference_main_runs_unchanged_on_our_packages(tmp_path, monkeypatch):
+    ref_main = write_reference_main(tmp_path)
     dropin = os.path.join(ROOT, "resilient-consensus-based-marl_b200")
     sys.path.insert(0, dropin)
     import run_main
@@ -29,7 +29,7 @@ def test_reference_main_runs_unchanged_on_our_packages(tmp_path, monkeypatch):
         return w, pd.DataFrame([{"True_team_returns": 0.0, "True_adv_returns": 0.0, "Estimated_team_returns": 0.0}])
     monkeypatch.setattr(training, "train_RPBCAC", fake_train)
     monkeypatch.chdir(tmp_path)                      # main.py writes its artefacts to the cwd (main.py:119-121)
-    run_main.main(["run_main.py", REF_MAIN, "--H=1", "--slow_lr=0.002", "--random_seed=100", "--n_episodes=50"])
+    run_main.main(["run_main.py", ref_main, "--H=1", "--slow_lr=0.002", "--random_seed=100", "--n_episodes=50"])
     from agents.resilient_CAC_agents import RPBCAC_agent
     from environments.grid_world import Grid_World
     assert type(seen["env"]) is Grid_World and seen["env"].__class__.__module__ == "environments.grid_world"

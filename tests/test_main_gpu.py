@@ -2,10 +2,8 @@
 end to end on the drop-in packages through REAL training on the GPU: argparse -> model / agent / env construction
 (main.py:59-116) -> training.train_RPBCAC (main.py:117) -> the three artefacts (main.py:119-121).  The driver comes out of
 tests/golden/ref_main_py.npz (a compressed blob written by oracle/make_golden.py; the GPU box has no reference checkout)."""
-import hashlib
 import os
 import sys
-import zlib
 
 import numpy as np
 import pandas as pd
@@ -14,7 +12,7 @@ import pytest
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
-from golden_util import load            # noqa: E402
+from golden_util import write_reference_main            # noqa: E402
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -24,11 +22,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def test_reference_main_trains_end_to_end_unchanged(n_envs, flags, tmp_path, monkeypatch, capsys):
     if not torch.cuda.is_available():
         pytest.skip("needs a CUDA device")
-    z = load("ref_main_py.npz")
-    raw = zlib.decompress(z["blob"].tobytes())
-    assert hashlib.sha256(raw).hexdigest() == str(z["sha256"]) and len(raw) == int(z["n_bytes"])
-    script = tmp_path / "main.py"
-    script.write_bytes(raw)
+    script = write_reference_main(tmp_path)
     dropin = os.path.join(ROOT, "resilient-consensus-based-marl_b200")
     sys.path.insert(0, dropin)
     import run_main

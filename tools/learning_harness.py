@@ -1,6 +1,6 @@
 """Learning-curve reproduction harness (SURVEY 8f.2, README.md:31-45 of the reference): every published run directory
 (8 scenarios x H in {0, 1} x seeds {100, 200, 300}; 45 exist) is re-run from ITS OWN start weights and task
-(tests/golden/ref_learning.npz, extracted by oracle/make_golden.py -- the GPU box needs no reference checkout), and the mean
+(tests/golden/ref_learning/<scenario>.npz, extracted by oracle/make_golden.py -- no reference checkout is needed), and the mean
 of the last 500 episodes is printed next to the mean of the last 500 episodes of the reference's sim_data2.pkl.
 
     python tools/learning_harness.py [n_blocks=40] [n_envs=256] [filter]      -> gpurun_out/learning_harness.{json,md}
@@ -26,11 +26,14 @@ from rcmarl.trainer import Trainer             # noqa: E402
 n_blocks = int(sys.argv[1]) if len(sys.argv) > 1 else 40
 n_envs = int(sys.argv[2]) if len(sys.argv) > 2 else 256
 only = sys.argv[3] if len(sys.argv) > 3 else ""
-z = np.load(os.path.join(ROOT, "tests", "golden", "ref_learning.npz"))
-runs = [str(r) for r in z["runs"] if only in str(r)]
+golden = os.path.join(ROOT, "tests", "golden", "ref_learning")
+runs = []                                       # (run tag, the scenario's fixture holding it)
+for name in sorted(os.listdir(golden)):
+    z = np.load(os.path.join(golden, name))
+    runs += [(str(r), z) for r in z["runs"] if only in str(r)]
 tail = 10                                       # 10 blocks x 50 episodes = the last 500 episodes
 rows = []
-for tag in runs:
+for tag, z in runs:
     scen, Hs, ss = tag.split("/")
     H, seed = int(Hs[1:]), int(ss[1:])
     labels = [str(x) for x in z[f"{tag}/labels"]]
