@@ -141,7 +141,9 @@ int rcmarl_values(const rcmarl_rows* rows_host, const rcmarl_value_job* jobs_hos
  * sums[j] = [ d(loss)/d(theta) (n_params) | loss ]   -- UNSCALED sums, so that a data-parallel
  * all-reduce can be applied before the division by the global batch size.
  * Replaces the forward/backward inside critic.fit / TR.fit / actor.train_on_batch / actor.fit
- * (agents/resilient_CAC_agents.py:99,118,136; adversarial:41,116,133,150,163,224,239,251). */
+ * (agents/resilient_CAC_agents.py:99,118,136; adversarial:41,116,133,150,163,224,239,251).
+ * max_ctas > 0 plans the grid within that many CTAs (one per SM) instead of the whole GPU (max_ctas = 0), so that other
+ * work can run beside it on the remaining SMs (rcmarl_overlap_split). */
 typedef enum { RCMARL_LOSS_MSE = 0, RCMARL_LOSS_CE = 1 } rcmarl_loss;
 typedef struct {
     const float* w;
@@ -154,7 +156,7 @@ typedef struct {
     int32_t action_agent;       /* CE only */
 } rcmarl_grad_job;
 int rcmarl_grad(const rcmarl_rows* rows_host, const rcmarl_grad_job* jobs_host, int n_jobs,
-                int loss_mode, void* ws, int64_t ws_bytes, void* stream);
+                int loss_mode, void* ws, int64_t ws_bytes, int max_ctas, void* stream);
 
 /* theta_dst = theta_src - coef * g   (plain SGD, Keras SGD(lr): coef = lr * 2/B for MSE)
  * loss_out (optional) = loss_coef * g[n]  -- history['loss'][0] bookkeeping. */
@@ -196,12 +198,25 @@ int rcmarl_minibatch_sgd(const rcmarl_rows* rows_host, const rcmarl_grad_job* gj
  *   cells / cells_bytes: caller-owned scratch of rcmarl_minibatch_cells_bytes() bytes that must be ZERO before the
  *     first call and is otherwise only touched by this entry point;
  *   seq_first >= 1: first of the `rcmarl_minibatch_steps()` consecutive sequence numbers this call consumes; the
- *     caller passes strictly increasing, non-overlapping ranges over the lifetime of `cells`. */
+ *     caller passes strictly increasing, non-overlapping ranges over the lifetime of `cells`;
+ *   max_ctas > 0: the chains share at most that many CTAs (cost-sized shares, as with the whole GPU at max_ctas = 0). */
 int64_t rcmarl_minibatch_cells_bytes(int n_jobs, int max_params);
 int64_t rcmarl_minibatch_steps(int epochs, int n_times, int mb_times);
 int rcmarl_minibatch_fit(const rcmarl_rows* rows_host, const rcmarl_grad_job* gjobs_host,
                          const rcmarl_sgd_job* sjobs_host, int n_jobs, int epochs, int n_times, int mb_times,
-                         float lr, void* cells, int64_t cells_bytes, uint32_t seq_first, void* stream);
+                         float lr, void* cells, int64_t cells_bytes, uint32_t seq_first, int max_ctas, void* stream);
+
+/* How an update round may split the GPU between the cooperative agents' full-batch fits (rcmarl_grad: n_fit jobs of kinds
+ * fit_kinds_host over fit_rows rows, fit_launches launches per epoch) and the adversaries' mini-batch chains
+ * (rcmarl_minibatch_fit: n_chains chains of kinds chain_kinds_host, mb_rows rows per SGD step, mb_steps steps per epoch)
+ * when the two run at the same time on two streams of one GPU with sm_count SMs.  budgets_host[0] = max_ctas for the
+ * fits, budgets_host[1] = max_ctas for the chains: they sum to at most sm_count, every job and chain gets at least one CTA
+ * and the fits' budget is a multiple of n_fit (equal shares).  Both 0: run the phases one after the other on the whole
+ * GPU -- when either is empty, world > 1, n_agents != 5 (no measured cost model) or the model predicts too little gain.
+ * Host arithmetic only (no device needed). */
+int rcmarl_overlap_split(int n_agents, const int32_t* fit_kinds_host, int n_fit, int64_t fit_rows, int fit_launches,
+                         const int32_t* chain_kinds_host, int n_chains, int64_t mb_rows, int64_t mb_steps, int world,
+                         int sm_count, int32_t* budgets_host);
 
 /* Keras/TF-2 Adam (SURVEY Appendix A.5): m,v updated in place, theta -= lr_t*m/(sqrt(v)+eps);
  * g = grad_scale * sums.  lr_t = lr*sqrt(1-b2^t)/(1-b1^t) is computed by the caller. */

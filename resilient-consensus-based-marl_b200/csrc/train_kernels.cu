@@ -614,10 +614,16 @@ static void plan_shares(int n, const int* cost, int64_t nchunks, int gw, int sms
     }
 }
 
-static int plan_grad_grid(GradParams& P, PartialSlots& S, const int* cost, int64_t nchunks, int gw) {
+// CTAs a launcher may plan with: the caller's budget (max_ctas > 0), at most the whole GPU (max_ctas = 0)
+static int cta_budget(int max_ctas) {
+    const int sms = sm_count_cached();
+    return max_ctas > 0 && max_ctas < sms ? max_ctas : sms;
+}
+
+static int plan_grad_grid(GradParams& P, PartialSlots& S, const int* cost, int64_t nchunks, int gw, int sms) {
     const int n = P.n_jobs;
     int g[RCMARL_MAX_JOBS];
-    plan_shares(n, cost, nchunks, gw, sm_count_cached(), balanced_grid_enabled(), g);
+    plan_shares(n, cost, nchunks, gw, sms, balanced_grid_enabled(), g);
     int first = 0;
     for (int j = 0; j < n; ++j) {
         P.cta_first[j] = (int16_t)first;
@@ -691,6 +697,28 @@ static int launch_mb_persist(const MbParams& P, int n_ctas, cudaStream_t st) {
     return 0;
 }
 
+// Cost model of rcmarl_overlap_split, per launch of a warp-specialised tensor-core kernel (n_agents = 5):
+//   time = fixed + per_tile * max over jobs of (128-row tiles of one CTA of the job * grad_row_cost of the job).
+// Constants from the round-2 measurements at the C2 shapes on one B200 (profiles/r02_kernel_experiments.md,
+// profiles/r02_bench_c2.json): rcmarl_grad over 12 288 000 rows x 8 jobs, 5.73 ms at 18 CTAs per job; a step of
+// rcmarl_minibatch_fit (3 chains x 131 072 rows), 39.2 us at 48 / 52 / 48 CTAs, of which ~11.6 us fixed tail.
+// tools/prof_overlap.py measures both at smaller budgets and refits them.  Running at the same time costs the two phases
+// some of each other's L2 and HBM bandwidth, which the model leaves out; kOverlapMinGain keeps them serial unless the
+// predicted saving clears that.
+static constexpr double kFitFixedNs = 30000.0, kFitTileNs = 0.494;     // rcmarl_grad: launch + reduce; ns per tile x cost
+static constexpr double kMbFixedNs = 11600.0, kMbTileNs = 0.61;        // one step of rcmarl_minibatch_fit: tail; sweep
+static constexpr double kOverlapMinGain = 0.02;
+
+// time of one launch in which job j sweeps `units` tiles with g[j] CTAs
+static double shares_time(int n, const int* cost, const int* g, int64_t units, double fixed_ns, double tile_ns) {
+    int64_t worst = 0;
+    for (int j = 0; j < n; ++j) {
+        const int64_t t = (units + g[j] - 1) / g[j] * cost[j];
+        if (t > worst) worst = t;
+    }
+    return fixed_ns + tile_ns * (double)worst;
+}
+
 }  // namespace rcmarl
 
 using namespace rcmarl;
@@ -719,6 +747,50 @@ int rcmarl_grad_grid_plan(int n_agents, const int32_t* kinds_host, int n_jobs, i
     return RCMARL_OK;
 }
 
+int rcmarl_overlap_split(int n_agents, const int32_t* fit_kinds_host, int n_fit, int64_t fit_rows, int fit_launches,
+                         const int32_t* chain_kinds_host, int n_chains, int64_t mb_rows, int64_t mb_steps, int world,
+                         int sm_count, int32_t* budgets_host) {
+    if ((n_agents != 5 && n_agents != 16) || !budgets_host || n_fit < 0 || n_fit > RCMARL_MAX_JOBS || n_chains < 0 ||
+        n_chains > RCMARL_MAX_JOBS || (n_fit && !fit_kinds_host) || (n_chains && !chain_kinds_host) || fit_rows < 0 ||
+        fit_launches < 0 || mb_rows < 0 || mb_steps < 0 || world < 1 || sm_count < 1)
+        return RCMARL_ERR_ARG;
+    int fit_cost[RCMARL_MAX_JOBS], mb_cost[RCMARL_MAX_JOBS], gf[RCMARL_MAX_JOBS], gm[RCMARL_MAX_JOBS];
+    for (int j = 0; j < n_fit; ++j) {
+        if (fit_kinds_host[j] < 0 || fit_kinds_host[j] > 2) return RCMARL_ERR_ARG;
+        fit_cost[j] = grad_job_cost(n_agents, fit_kinds_host[j], RCMARL_LOSS_MSE);
+    }
+    for (int j = 0; j < n_chains; ++j) {
+        if (chain_kinds_host[j] < 0 || chain_kinds_host[j] > 2) return RCMARL_ERR_ARG;
+        mb_cost[j] = grad_job_cost(n_agents, chain_kinds_host[j], RCMARL_LOSS_MSE);
+    }
+    budgets_host[0] = budgets_host[1] = 0;
+    // serial: nothing to overlap; the 16-agent kernels are not covered by the cost model; with world > 1 both phases would
+    // draw sequence numbers from the one cell region of the peer-memory exchange, whose call order must match on every rank
+    if (n_fit == 0 || n_chains == 0 || fit_rows == 0 || fit_launches == 0 || mb_rows == 0 || mb_steps == 0 ||
+        n_agents != 5 || world > 1 || sm_count < n_fit + n_chains)
+        return RCMARL_OK;
+    const int cpc = grad_chunks_per_cta<5>(RCMARL_LOSS_MSE);
+    const int64_t fit_chunks = (fit_rows + 63) / 64, mb_chunks = (mb_rows + 63) / 64;
+    const int64_t fit_units = (fit_chunks + cpc - 1) / cpc, mb_units = (mb_chunks + cpc - 1) / cpc;
+    auto fit_ns = [&](int ctas) {
+        plan_shares(n_fit, fit_cost, fit_chunks, cpc, ctas, false, gf);
+        return (double)fit_launches * shares_time(n_fit, fit_cost, gf, fit_units, kFitFixedNs, kFitTileNs);
+    };
+    auto mb_ns = [&](int ctas) {
+        plan_shares(n_chains, mb_cost, mb_chunks, cpc, ctas, true, gm);
+        return (double)mb_steps * shares_time(n_chains, mb_cost, gm, mb_units, kMbFixedNs, kMbTileNs);
+    };
+    const double serial = fit_ns(sm_count) + mb_ns(sm_count);
+    double best = serial;
+    // equal shares: only multiples of n_fit are worth giving the fits; the chains take every other CTA
+    for (int f = n_fit; f <= sm_count - n_chains; f += n_fit) {
+        const double t = fit_ns(f) > mb_ns(sm_count - f) ? fit_ns(f) : mb_ns(sm_count - f);
+        if (t < best) { best = t; budgets_host[0] = f; budgets_host[1] = sm_count - f; }
+    }
+    if (best > serial * (1.0 - kOverlapMinGain)) budgets_host[0] = budgets_host[1] = 0;
+    return RCMARL_OK;
+}
+
 int rcmarl_values(const rcmarl_rows* rows, const rcmarl_value_job* jobs, int n_jobs, void* stream) {
     if (int e = check_rows(rows)) return e;
     if (!jobs || n_jobs < 1 || n_jobs > RCMARL_MAX_JOBS) return RCMARL_ERR_ARG;
@@ -738,9 +810,9 @@ int rcmarl_values(const rcmarl_rows* rows, const rcmarl_value_job* jobs, int n_j
 }
 
 int rcmarl_grad(const rcmarl_rows* rows, const rcmarl_grad_job* jobs, int n_jobs, int loss_mode, void* ws,
-                int64_t ws_bytes, void* stream) {
+                int64_t ws_bytes, int max_ctas, void* stream) {
     if (int e = check_rows(rows)) return e;
-    if (!jobs || n_jobs < 1 || n_jobs > RCMARL_MAX_JOBS || !ws) return RCMARL_ERR_ARG;
+    if (!jobs || n_jobs < 1 || n_jobs > RCMARL_MAX_JOBS || !ws || max_ctas < 0) return RCMARL_ERR_ARG;
     if (loss_mode != RCMARL_LOSS_MSE && loss_mode != RCMARL_LOSS_CE) return RCMARL_ERR_ARG;
     const int NA = rows->n_agents;
     GradParams P;
@@ -768,7 +840,7 @@ int rcmarl_grad(const rcmarl_rows* rows, const rcmarl_grad_job* jobs, int n_jobs
     P.n_jobs = n_jobs;
     P.stride = maxn;
     Q.slots.stride = maxn;
-    const int n_ctas = plan_grad_grid(P, Q.slots, cost, nchunks, cpc);
+    const int n_ctas = plan_grad_grid(P, Q.slots, cost, nchunks, cpc, cta_budget(max_ctas));
     if ((int64_t)n_ctas * maxn * (int64_t)sizeof(float) > ws_bytes) return RCMARL_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     int e = NA == 5 ? launch_grad<5>(P, loss_mode, n_ctas, st) : launch_grad<16>(P, loss_mode, n_ctas, st);
@@ -824,7 +896,7 @@ int rcmarl_minibatch_sgd(const rcmarl_rows* rows, const rcmarl_grad_job* gjobs, 
             const int64_t n_rows = (int64_t)cnt * rows->n_envs;
             P.rows.n_rows = n_rows;
             if (cnt != planned_cnt) {                        // the grid only depends on the mini-batch size
-                n_ctas = plan_grad_grid(P, Q.slots, cost, (n_rows + 63) / 64, cpc);
+                n_ctas = plan_grad_grid(P, Q.slots, cost, (n_rows + 63) / 64, cpc, sm_count_cached());
                 if ((int64_t)n_ctas * maxn * (int64_t)sizeof(float) > ws_bytes) return RCMARL_ERR_WORKSPACE;
                 planned_cnt = cnt;
             }
@@ -869,11 +941,11 @@ int64_t rcmarl_minibatch_steps(int epochs, int n_times, int mb_times) {
 
 int rcmarl_minibatch_fit(const rcmarl_rows* rows, const rcmarl_grad_job* gjobs, const rcmarl_sgd_job* sjobs, int n_jobs,
                          int epochs, int n_times, int mb_times, float lr, void* cells, int64_t cells_bytes,
-                         uint32_t seq_first, void* stream) {
+                         uint32_t seq_first, int max_ctas, void* stream) {
     if (!rows || !rows->sa || !rows->ns || !rows->r || rows->n_envs <= 0) return RCMARL_ERR_ARG;
     if (rows->n_agents != 5 && rows->n_agents != 16) return RCMARL_ERR_ARG;
     if (!gjobs || !sjobs || n_jobs < 1 || n_jobs > RCMARL_MAX_JOBS || !cells || epochs < 1 || n_times < 1 || mb_times < 1 ||
-        seq_first < 1)
+        seq_first < 1 || max_ctas < 0)
         return RCMARL_ERR_ARG;
     const int NA = rows->n_agents;
     MbParams P;
@@ -910,7 +982,7 @@ int rcmarl_minibatch_fit(const rcmarl_rows* rows, const rcmarl_grad_job* gjobs, 
     int n_ctas = 0;
     {
         int g[RCMARL_MAX_JOBS];
-        plan_shares(n_jobs, cost, (n_rows_mb + 63) / 64, cpc, sm_count_cached(), true, g);
+        plan_shares(n_jobs, cost, (n_rows_mb + 63) / 64, cpc, cta_budget(max_ctas), true, g);
         for (int j = 0; j < n_jobs; ++j) { P.cta_first[j] = (int16_t)n_ctas; n_ctas += g[j]; }
         P.cta_first[n_jobs] = (int16_t)n_ctas;
     }

@@ -86,7 +86,7 @@ SYMBOLS = [
     ("rcmarl_clip_mean", C.c_int, [c_fp, C.c_int, C.c_int64, C.c_int64, C.c_int, c_fp, c_fp]),
     ("rcmarl_consensus_hidden", C.c_int, [C.POINTER(ConsensusJob), C.c_int, c_fp]),
     ("rcmarl_values", C.c_int, [C.POINTER(Rows), C.POINTER(ValueJob), C.c_int, c_fp]),
-    ("rcmarl_grad", C.c_int, [C.POINTER(Rows), C.POINTER(GradJob), C.c_int, C.c_int, c_fp, C.c_int64, c_fp]),
+    ("rcmarl_grad", C.c_int, [C.POINTER(Rows), C.POINTER(GradJob), C.c_int, C.c_int, c_fp, C.c_int64, C.c_int, c_fp]),
     ("rcmarl_sgd_apply", C.c_int, [C.POINTER(SgdJob), C.c_int, c_fp]),
     ("rcmarl_adam_apply", C.c_int, [C.POINTER(AdamJob), C.c_int, c_fp]),
     ("rcmarl_minibatch_sgd", C.c_int, [C.POINTER(Rows), C.POINTER(GradJob), C.POINTER(SgdJob), C.c_int, C.c_int, C.c_int,
@@ -94,7 +94,9 @@ SYMBOLS = [
     ("rcmarl_minibatch_cells_bytes", C.c_int64, [C.c_int, C.c_int]),
     ("rcmarl_minibatch_steps", C.c_int64, [C.c_int, C.c_int, C.c_int]),
     ("rcmarl_minibatch_fit", C.c_int, [C.POINTER(Rows), C.POINTER(GradJob), C.POINTER(SgdJob), C.c_int, C.c_int, C.c_int,
-                                       C.c_int, C.c_float, c_fp, C.c_int64, C.c_uint32, c_fp]),
+                                       C.c_int, C.c_float, c_fp, C.c_int64, C.c_uint32, C.c_int, c_fp]),
+    ("rcmarl_overlap_split", C.c_int, [C.c_int, C.POINTER(C.c_int32), C.c_int, C.c_int64, C.c_int, C.POINTER(C.c_int32),
+                                       C.c_int, C.c_int64, C.c_int64, C.c_int, C.c_int, C.POINTER(C.c_int32)]),
     ("rcmarl_team", C.c_int, [C.POINTER(Rows), C.POINTER(TeamJob), C.c_int, c_fp, C.c_int64, c_fp]),
     ("rcmarl_reward_mix", C.c_int, [c_fp, C.c_int64, C.c_int, C.POINTER(C.c_int32), C.c_int, C.c_float, c_fp, c_fp]),
     ("rcmarl_comm_create", C.c_int, [C.c_int, C.c_int, C.c_int64, C.POINTER(C.c_void_p)]),

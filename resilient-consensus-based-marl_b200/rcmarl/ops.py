@@ -118,11 +118,12 @@ def grad_job(w, target, sums, kind, action_agent=0, target_stride=1, time_idx=No
     return j
 
 
-def grad(rows, jobs, loss_mode, ws=None):
+def grad(rows, jobs, loss_mode, ws=None, max_ctas=0):
+    """max_ctas > 0: plan the grid within that many CTAs (the rest of the GPU stays free for another stream)."""
     a = jobs if isinstance(jobs, C.Array) else _arr(L.GradJob, jobs)
     if ws is None:
         ws = workspace()
-    L.check(L.lib().rcmarl_grad(C.byref(rows), a, len(a), loss_mode, ws.data_ptr(), ws.numel(), _stream()),
+    L.check(L.lib().rcmarl_grad(C.byref(rows), a, len(a), loss_mode, ws.data_ptr(), ws.numel(), max_ctas, _stream()),
             "rcmarl_grad")
 
 
@@ -161,8 +162,9 @@ class MinibatchCells:
         self.seq = 1
 
 
-def minibatch_fit(rows, gjobs, sjobs, epochs, n_times, mb_times, lr, cells):
-    """Whole mini-batch fit (all epochs, all steps, all chains) as ONE persistent kernel (csrc/minibatch_persist.cuh)."""
+def minibatch_fit(rows, gjobs, sjobs, epochs, n_times, mb_times, lr, cells, max_ctas=0):
+    """Whole mini-batch fit (all epochs, all steps, all chains) as ONE persistent kernel (csrc/minibatch_persist.cuh);
+    max_ctas > 0: the chains share at most that many CTAs."""
     ga = gjobs if isinstance(gjobs, C.Array) else _arr(L.GradJob, gjobs)
     sa = sjobs if isinstance(sjobs, C.Array) else _arr(L.SgdJob, sjobs)
     steps = L.lib().rcmarl_minibatch_steps(epochs, n_times, mb_times)
@@ -170,9 +172,20 @@ def minibatch_fit(rows, gjobs, sjobs, epochs, n_times, mb_times, lr, cells):
         cells.buf.zero_()
         cells.seq = 1
     L.check(L.lib().rcmarl_minibatch_fit(C.byref(rows), ga, sa, len(ga), epochs, n_times, mb_times, lr,
-                                         cells.buf.data_ptr(), cells.buf.numel(), cells.seq, _stream()),
+                                         cells.buf.data_ptr(), cells.buf.numel(), cells.seq, max_ctas, _stream()),
             "rcmarl_minibatch_fit")
     cells.seq += steps
+
+
+def overlap_split(n_agents, fit_kinds, fit_rows, fit_launches, chain_kinds, mb_rows, mb_steps, world, sm_count):
+    """(CTAs for the full-batch fits, CTAs for the mini-batch chains) when the two run at the same time on two streams,
+    or None: run them one after the other on the whole GPU (rcmarl_overlap_split)."""
+    fk = (C.c_int32 * max(len(fit_kinds), 1))(*fit_kinds)
+    ck = (C.c_int32 * max(len(chain_kinds), 1))(*chain_kinds)
+    out = (C.c_int32 * 2)()
+    L.check(L.lib().rcmarl_overlap_split(n_agents, fk, len(fit_kinds), fit_rows, fit_launches, ck, len(chain_kinds),
+                                         mb_rows, mb_steps, world, sm_count, out), "rcmarl_overlap_split")
+    return (out[0], out[1]) if out[0] else None
 
 
 def adam_job(theta, m, v, sums, n, grad_scale, lr_t, beta1=0.9, beta2=0.999, eps=1e-7, loss_out=None, loss_coef=0.0,

@@ -121,6 +121,7 @@ class Trainer:
         self.mb_cells = None
         if os.environ.get("RCMARL_MB_PERSIST", "1") != "0":
             self.mb_cells = ops.MinibatchCells(L.MAX_JOBS, self.PT if NA == 5 else L.param_count(48, 1), self.dev)
+        self._side = None                                 # stream of the mini-batch chains when they overlap the fits
         self.launches = 0                                 # kernels launched by this engine (bench: gpu_launches)
         self.profile = None                               # bench.py: {"fit_grad": [(start_evt, end_evt), ...], ...}
         self.h2d_bytes = 4 * sum(x.numel() for x in (self.actor, self.critic, self.tr, self.critic_local))
@@ -321,6 +322,18 @@ class Trainer:
                 chains.append((self.tr[i], L.IN_SA, r_col[i], NA, self.loss_t[i:i + 1], lr_i))
                 chains.append((self.critic[i], L.IN_S, self.tdt[i], 1, self.loss_c[i:i + 1], lr_i))
 
+        # The chains and the cooperative fits touch disjoint parameters and scratch and only read the buffer and the TD
+        # targets, so they may run at the same time on two streams, each on its share of the SMs (rcmarl_overlap_split).
+        fit_ctas = mb_ctas = 0
+        if coop and chains and self.mb_cells is not None:
+            split = ops.overlap_split(NA, [j.kind for j in fit_first], B, self.local_steps, [ch[1] for ch in chains],
+                                      self.mb_times * N, self.mb_epochs * ((T + self.mb_times - 1) // self.mb_times),
+                                      self.world, torch.cuda.get_device_properties(self.dev).multi_processor_count)
+            if split is not None:
+                fit_ctas, mb_ctas = split
+                if self._side is None:
+                    self._side = torch.cuda.Stream(self.dev, priority=-1)
+
         cons_jobs, team_jobs, team_apply = [], [], []
         for n, i in enumerate(coop):
             nodes = self.in_nodes[i]
@@ -337,13 +350,23 @@ class Trainer:
             if td_arr is not None:
                 ops.values(rows_all, td_arr)
                 self.launches += 1
+            if mb_ctas:                                                    # chains first: the side stream has priority
+                fork, join = torch.cuda.Event(), torch.cuda.Event()
+                fork.record()
+                self._side.wait_event(fork)
+                with torch.cuda.stream(self._side):                        # perms are allocated on this stream
+                    self._timed("minibatch_sgd", self._minibatch_sgd, chains, T, mb_ctas)
+                    join.record()
             if coop:
                 for step in range(self.local_steps):                      # fit(batch_size=B, epochs=5), res..py:118,136
-                    self._timed("fit_grad", ops.grad, rows_all, fit_first if step == 0 else fit_next, L.LOSS_MSE, self.ws)
+                    self._timed("fit_grad", ops.grad, rows_all, fit_first if step == 0 else fit_next, L.LOSS_MSE, self.ws,
+                                fit_ctas)
                     self._allreduce(self.sums_fit[:2 * len(coop)])
                     ops.sgd_apply(fit_apply_first if step == 0 else fit_apply_next)
                     self.launches += 3
-            if chains:
+            if mb_ctas:
+                torch.cuda.current_stream().wait_event(join)
+            elif chains:
                 self._timed("minibatch_sgd", self._minibatch_sgd, chains, T)
             for i in range(self.n_real):                                   # the transmitted messages (:118-121)
                 if lab[i] != COOP:
@@ -399,7 +422,7 @@ class Trainer:
         self.trim()
         return losses
 
-    def _minibatch_sgd(self, chains, T):
+    def _minibatch_sgd(self, chains, T, max_ctas=0):
         """10 epochs x ceil(T/32) sequential SGD steps per chain; a mini-batch = 32 time rows x all environments
         (Appendix C).  All chains advance in lock-step: one grad launch + one apply launch per step."""
         N, nb = self.N, (T + self.mb_times - 1) // self.mb_times
@@ -428,7 +451,7 @@ class Trainer:
             if self.mb_cells is not None:                   # one persistent kernel for the whole fit
                 for c in range(nC):
                     aj[c].coef = lrs[c]                     # per-chain learning rate
-                ops.minibatch_fit(rows, gj, aj, E, T, self.mb_times, lrs[0], self.mb_cells)
+                ops.minibatch_fit(rows, gj, aj, E, T, self.mb_times, lrs[0], self.mb_cells, max_ctas)
                 self.launches += 1
                 return
             if len(set(lrs)) != 1:
